@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the BASELINE.json metric: Flow.log_prob samples/s on the 10-layer RQ-NSF, D=784, batch 2^20, sharded over N GPUs.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--rows R] [--weak]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--rows R] [--weak] [--dump-outputs DIR]
 
 One "step" = one Flow.log_prob pass over ONE synthetic Gaussian batch of R rows (default 2^20, BASELINE.json configs[2]).
 With N GPUs (torchrun, one rank per GPU) the batch is SHARDED: every rank owns R/N rows and a replica of the weights
@@ -276,6 +276,19 @@ def extra_workloads(dev, flow):
     return out
 
 
+def dump_outputs(directory, log_prob, limit_bytes=64 << 20):
+    """Writes the per-sample log-probs as DIR/log_prob.npy (float32).  An output over `limit_bytes` is replaced by a fixed,
+    seeded sample of rows, whose indices go to DIR/log_prob_rows.npy (float64, exact for any row count)."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    lp = log_prob.float().cpu()
+    if lp.numel() * 4 > limit_bytes:
+        rows = torch.randperm(lp.numel(), generator=torch.Generator().manual_seed(0))[:limit_bytes // 12].sort().values
+        lp = lp[rows]
+        np.save(os.path.join(directory, "log_prob_rows.npy"), rows.double().numpy())
+    np.save(os.path.join(directory, "log_prob.npy"), lp.numpy())
+
+
 def run_reference(args):
     """--impl reference: the reference's CPU path (oracle port; the Python reference itself cannot travel to the GPU box), on
     ALL host threads -- torchrun exports OMP_NUM_THREADS=1, undone here; ranks other than 0 exit without work."""
@@ -360,6 +373,7 @@ def run_native(args):
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         ms_total = float(ms.item())
         lp_local = out[rank * rows:(rank + 1) * rows].clone() if world > 1 else out.clone()
+        last_out = out.cpu() if args.dump_outputs and rank == 0 else None
 
         # ---- end to end: pinned host inputs -> H2D -> log_prob -> D2H of the result, every step ------------------
         host_x = torch.empty(rows, FEATURES, pin_memory=True)
@@ -474,6 +488,8 @@ def run_native(args):
         result["cpu_baseline"] = {"value": rate, "unit": "samples/s", "cores": threads, "kind": "port",
                                   "sample": "%d rows of the same workload in chunks of 2048" % sample_rows}
     print(json.dumps(result))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_out)
     if world > 1:
         dist.destroy_process_group()
     if "parity_check" in result and not result["parity_check"]["ok"]:
@@ -497,7 +513,12 @@ def main():
     ap.add_argument("--block-rows", type=int, default=0, help="override config.{trunk,affine,coupling}_block_rows (experiments)")
     ap.add_argument("--no-spline-roofline", action="store_true")
     ap.add_argument("--e2e-chunk", type=int, default=1 << 17, help="rows per host->device chunk of the end-to-end leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the log-probs of the last timed step to DIR/log_prob.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs applies to --impl native")
     if args.block_rows:
         from nflows_b200 import config
         config.trunk_block_rows = config.affine_block_rows = config.coupling_block_rows = args.block_rows
