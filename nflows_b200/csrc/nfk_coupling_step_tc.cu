@@ -14,8 +14,8 @@
 //     reads back exactly what it wrote).
 //
 // Arithmetic is that of nfk_linear_tc.cu / nfk_rq_coupling_tc.cu: fp16 split pairs with power-of-two scales, three
-// kind::f16 MMAs per K-step, partial sums of 2 (trunk) / 4 (final layer) K-slabs drained from TMEM and accumulated in
-// registers with round-to-nearest adds.
+// kind::f16 MMAs per K-step, partial sums of STEP_DRAIN_TRUNK = 4 (trunk) / STEP_DRAIN_FINAL = 8 (final layer) K-slabs
+// drained from TMEM and accumulated in registers with round-to-nearest adds.
 //
 // Shared memory (dynamic, 1024-aligned):
 //   [0, 128 KB)        R
@@ -26,7 +26,6 @@
 //        G2 final layer   : 3 stages x 24 KB [W hi | W lo] of one K-slab x one column tile (BN <= 192)
 //   then barriers, log|det| partials, packed-bias double buffer, 3 output staging buffers.
 // TMEM: 2 partial accumulators x 256 columns.
-#include <stdlib.h>
 #include <string.h>
 
 #include "fused_spline.cuh"
@@ -40,8 +39,8 @@ constexpr int STEP_MAX_LAYERS = 9;                                   // initial 
 // Final layer (spline logits, insensitive): the whole K = 256 in one partial sum; trunk layers: K = 128 per partial sum.
 // Measured (cfg 3, 2^20 rows, parity_check of bench.py against the CPU oracle): final 4 -> 8: 182 -> 175 ms in this kernel,
 // rel. error 2.2e-6 -> 2.4e-6; trunk 2 -> 4: -2 ms, unchanged error (profiles/drain_sweep_r2.txt).
-constexpr int STEP_DRAIN_FINAL_DEFAULT = 8;
-constexpr int STEP_DRAIN_TRUNK_DEFAULT = 4;
+constexpr int STEP_DRAIN_FINAL = 8;
+constexpr int STEP_DRAIN_TRUNK = 4;
 constexpr int STEP_SLAB_BYTES = 2 * A_BYTES;                         // one K-slab of R: hi | lo
 constexpr int STEP_R_BYTES = (BN_MAX / BK) * STEP_SLAB_BYTES;        // 128 KB
 constexpr int STEP_RING_BYTES = 80 * 1024;
@@ -108,14 +107,7 @@ struct StepParams {
     float* y;
     const int32_t* t_cols;
     int t_col0, tma_y, pair_only;
-    int mma_warps;                // 2: two MMA-issuing warps take alternate partial sums; 1: one issuer
-    int drain_t;                  // K-slabs accumulated in TMEM per partial sum of a trunk layer (DRAIN_SLABS_LINEAR by default)
-    int drain_f;                  // K-slabs accumulated in TMEM per partial sum of the final layer (DRAIN_SLABS_FUSED, or all)
     uint32_t zero;                // always 0 (mbar_arrive_after_loads)
-    int x_prefetch;               // NFK_STEP_X_PREFETCH=1: TMA-prefetch a row block's input tiles into L2 before its final phase
-    int k16;                      // NFK_STEP_K16=1 (experiment, off): final-layer weights stream as SIX stages of one K = 16 step each
-                                  // (SWIZZLE_32B rows) instead of three K = 32 slabs -- same 72 KB of ring, 5/6 instead of 2/3 of it in
-                                  // flight; correct, but 9 % slower (32-byte TMA rows / twice the barrier traffic)
     int tma_x;                    // inputs of the transformed features arrive as TMA boxes (consecutive columns, 16-byte aligned)
     float out_scale;
     float* lad_accum;
@@ -171,10 +163,10 @@ rq_coupling_step_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __gr
     const int warp = tid_x >> 5, lane = tid_x & 31;
     const int num_k0 = (p.K0 + BK - 1) / BK;                 // K-slabs of the initial layer
     const int num_kh = p.H / BK;                             // K-slabs of every other layer (H is a multiple of 32)
-    const int drain_t = p.drain_t;                           // K-slabs per partial sum of a trunk layer
+    constexpr int drain_t = STEP_DRAIN_TRUNK;                // K-slabs per partial sum of a trunk layer
     const int groups0 = (num_k0 + drain_t - 1) / drain_t;
     const int groupsh = (num_kh + drain_t - 1) / drain_t;
-    const int drain_f = p.drain_f;                           // K-slabs per partial sum of the final layer
+    constexpr int drain_f = STEP_DRAIN_FINAL;                // K-slabs per partial sum of the final layer
     const int groupsf = (num_kh + drain_f - 1) / drain_f;
     const int nch = p.H > 128 ? 2 : 1;                       // column chunks of a square layer
     const int ch = p.H / nch;                                // columns per chunk (multiple of 16)
@@ -284,14 +276,6 @@ rq_coupling_step_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __gr
                         continue;
                     }
                     // ---- G2: final layer, one stage = one K-slab of one column tile
-                    if (p.tma_x && p.x_prefetch) {
-                        // the row block's input tiles towards L2 now (each is 128 separate 32-byte row segments of HBM): their TMA
-                        // loads below then hit L2 instead of sitting in the TMA queue in front of the weight stages for a DRAM latency
-                        for (int n = 0; n < p.num_n_tiles; ++n)
-                            asm volatile("cp.async.bulk.prefetch.tensor.2d.L2.global.tile [%0, {%1, %2}];" ::"l"(reinterpret_cast<uint64_t>(&map_x)),
-                                         "r"(p.t_col0 + n * TF), "r"(m0)
-                                         : "memory");
-                    }
                     drain();
                     {
                         constexpr uint32_t tx = 2u * (uint32_t)BN * ROW_BYTES;
@@ -313,26 +297,6 @@ rq_coupling_step_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __gr
                                              bar_bfull + 8 * bslot);
                                 if (++bslot == 2) { bslot = 0; bphase ^= 1; }
                             }
-                            if (p.k16) {
-                                // six half-slab stages: [BN rows][32 bytes] hi, then lo (6 KB each at BN = 192)
-                                for (int kh = 0; kh < 2 * num_kh; ++kh) {
-                                    slot_wait(s);
-                                    const uint32_t full = bar_full + 8 * s;
-                                    const uint32_t sw = ring + s * (STEP_G2_STAGE_BYTES / 2);
-                                    mbar_expect_tx(full, tx / 2);
-                                    if (CL == 1) {
-                                        tma_load_2d(sw, &map_wf_hi, full, kh * 16, n * BN);
-                                        tma_load_2d(sw + BN * 32, &map_wf_lo, full, kh * 16, n * BN);
-                                    } else {
-                                        const uint32_t off = (uint32_t)(cta_rank * wrows) * 32u;
-                                        tma_load_2d_multicast(sw + off, &map_wf_hi, full, kh * 16, n * BN + cta_rank * wrows, cl_mask);
-                                        tma_load_2d_multicast(sw + BN * 32 + off, &map_wf_lo, full, kh * 16, n * BN + cta_rank * wrows, cl_mask);
-                                    }
-                                    uses ^= 1u << s;
-                                    if (++s == 2 * STEP_G2_STAGES) s = 0;
-                                }
-                                continue;
-                            }
                             for (int ks = 0; ks < num_kh; ++ks) {
                                 slot_wait(s);
                                 const uint32_t full = bar_full + 8 * s;
@@ -353,26 +317,13 @@ rq_coupling_step_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __gr
                     }
                 }
             }
-        } else if (warp == 1 || (warp == 3 && p.mma_warps == 2)) {
-            // ================================================= MMA issuers (one elected thread per issuing warp).
-            // TWO issuing warps take alternate partial sums (warp 1: TMEM buffer 0, warp 3: buffer 1): what limited the tensor
-            // pipe was the issue sequence itself -- every tcgen05.mma is preceded by an ELECT and five R2UR moves of its
-            // descriptors into uniform registers, ~190 cycles per instruction against 96 cycles of tensor work at N = 192 (ncu r2:
-            // the issuing warp never waited on a barrier, tensor pipe 50 %).  The MMAs of one partial sum come from one warp, in
-            // program order, so results do not depend on how the two warps interleave.
-            if (elect_one()) {                                       // ONE elected thread runs the role (uniform datapath)
-            const bool leader = true;
-            const int my = warp == 1 ? 0 : 1;
-            const bool solo = p.mma_warps != 2;
+        } else if (warp == 1) {
+            // ================================================= MMA issuer (one elected thread: uniform datapath, see elect_one)
+            if (elect_one()) {
             uint32_t seen = 0;                                       // bit s: parity of the number of fills of ring slot s consumed
             auto full_wait = [&](int s) { mbar_wait(bar_full + 8 * s, (seen >> s) & 1u); seen ^= 1u << s; };
             auto release = [&](int s) {
-                if (!leader) return;
                 if (CL == 1) umma_commit(bar_empty + 8 * s); else umma_commit_multicast(bar_empty + 8 * s, cl_mask);
-            };
-            // the other warp's partial sum: step over its ring slots (slot parities stay in step with the barriers)
-            auto pass = [&](int& s, int count, int stages) {
-                for (int j = 0; j < count; ++j) { seen ^= 1u << s; if (++s == stages) s = 0; }
             };
             const uint32_t idesc0 = make_idesc(p.H), idesc1 = make_idesc(ch), idescf = make_idesc(BN);
             uint32_t gc = 0;                                         // partial sums so far: buffer gc & 1, use (gc >> 1) of it
@@ -383,7 +334,6 @@ rq_coupling_step_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __gr
                     int s = 0;
                     for (int g = 0; g < groups0; ++g, ++gc) {
                         const int slabs = min(drain_t, num_k0 - g * drain_t);
-                        if (!solo && (int)(gc & 1u) != my) { pass(s, slabs, STEP_G0_STAGES); continue; }
                         const int acc = gc & 1u;
                         mbar_wait(bar_tempty + 8 * acc, ((gc >> 1) & 1u) ^ 1u);
                         const uint32_t d_tmem = tmem_base + acc * BN_MAX;
@@ -396,18 +346,18 @@ rq_coupling_step_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __gr
 #pragma unroll
                             for (int kk = 0; kk < BK / 16; ++kk) {
                                 const uint64_t adv = (uint64_t)(kk * 2);
-                                if (leader) umma_f16(d_tmem, a_lo + adv, w_hi + adv, idesc0, (j | kk) != 0);
-                                if (leader) umma_f16(d_tmem, a_hi + adv, w_lo + adv, idesc0, 1);
+                                umma_f16(d_tmem, a_lo + adv, w_hi + adv, idesc0, (j | kk) != 0);
+                                umma_f16(d_tmem, a_hi + adv, w_lo + adv, idesc0, 1);
                             }
 #pragma unroll
                             for (int kk = 0; kk < BK / 16; ++kk) {
                                 const uint64_t adv = (uint64_t)(kk * 2);
-                                if (leader) umma_f16(d_tmem, a_hi + adv, w_hi + adv, idesc0, 1);
+                                umma_f16(d_tmem, a_hi + adv, w_hi + adv, idesc0, 1);
                             }
                             release(s);
                             if (++s == STEP_G0_STAGES) s = 0;
                         }
-                        if (leader) umma_commit(bar_tfull + 8 * acc);
+                        umma_commit(bar_tfull + 8 * acc);
                     }
                 }
                 // ---- square layers: A from R, W from the G1 units
@@ -419,7 +369,6 @@ rq_coupling_step_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __gr
                         tc_fence_after();
                         for (int g = 0; g < groupsh; ++g, ++gc) {
                             const int slabs = min(drain_t, num_kh - g * drain_t);
-                            if (!solo && (int)(gc & 1u) != my) { pass(s, slabs * nch, STEP_G1_UNITS); continue; }
                             const int acc = gc & 1u;
                             mbar_wait(bar_tempty + 8 * acc, ((gc >> 1) & 1u) ^ 1u);
                             for (int c = 0; c < nch; ++c) {
@@ -434,19 +383,19 @@ rq_coupling_step_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __gr
 #pragma unroll
                                     for (int kk = 0; kk < BK / 16; ++kk) {
                                         const uint64_t adv = (uint64_t)(kk * 2);
-                                        if (leader) umma_f16(d_tmem, a_lo + adv, w_hi + adv, idesc1, (j | kk) != 0);
-                                        if (leader) umma_f16(d_tmem, a_hi + adv, w_lo + adv, idesc1, 1);
+                                        umma_f16(d_tmem, a_lo + adv, w_hi + adv, idesc1, (j | kk) != 0);
+                                        umma_f16(d_tmem, a_hi + adv, w_lo + adv, idesc1, 1);
                                     }
 #pragma unroll
                                     for (int kk = 0; kk < BK / 16; ++kk) {
                                         const uint64_t adv = (uint64_t)(kk * 2);
-                                        if (leader) umma_f16(d_tmem, a_hi + adv, w_hi + adv, idesc1, 1);
+                                        umma_f16(d_tmem, a_hi + adv, w_hi + adv, idesc1, 1);
                                     }
                                     release(s);
                                     if (++s == STEP_G1_UNITS) s = 0;
                                 }
                             }
-                            if (leader) umma_commit(bar_tfull + 8 * acc);
+                            umma_commit(bar_tfull + 8 * acc);
                         }
                     }
                 }
@@ -462,29 +411,9 @@ rq_coupling_step_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __gr
                     for (int n = 0; n < p.num_n_tiles; ++n) {
                         for (int g = 0; g < groupsf; ++g, ++gc) {
                             const int slabs = min(drain_f, num_kh - g * drain_f);
-                            if (!solo && (int)(gc & 1u) != my) { pass(s, p.k16 ? 2 * slabs : slabs, p.k16 ? 2 * STEP_G2_STAGES : STEP_G2_STAGES); continue; }
                             const int acc = gc & 1u;
                             mbar_wait(bar_tempty + 8 * acc, ((gc >> 1) & 1u) ^ 1u);
                             const uint32_t d_tmem = tmem_base + acc * BN_MAX;
-                            if (p.k16) {
-                                // one stage per K = 16 step: cross terms, main product, release
-                                for (int j = 0; j < 2 * slabs; ++j) {
-                                    full_wait(s);
-                                    tc_fence_after();
-                                    const uint32_t sa = smem_base + (g * drain_f + (j >> 1)) * STEP_SLAB_BYTES;
-                                    const uint32_t sw = ring + s * (STEP_G2_STAGE_BYTES / 2);
-                                    const uint64_t adv = (uint64_t)((j & 1) * 2);          // second K step of the resident 64-byte rows
-                                    const uint64_t a_hi = make_smem_desc(sa) + adv, a_lo = make_smem_desc(sa + A_BYTES) + adv;
-                                    const uint64_t w_hi = make_smem_desc_k16(sw), w_lo = make_smem_desc_k16(sw + BN * 32);
-                                    if (leader) umma_f16(d_tmem, a_lo, w_hi, idescf, j != 0);
-                                    if (leader) umma_f16(d_tmem, a_hi, w_lo, idescf, 1);
-                                    if (leader) umma_f16(d_tmem, a_hi, w_hi, idescf, 1);
-                                    release(s);
-                                    if (++s == 2 * STEP_G2_STAGES) s = 0;
-                                }
-                                if (leader) umma_commit(bar_tfull + 8 * acc);
-                                continue;
-                            }
                             for (int j = 0; j < slabs; ++j) {
                                 full_wait(s);
                                 tc_fence_after();
@@ -495,18 +424,18 @@ rq_coupling_step_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __gr
 #pragma unroll
                                 for (int kk = 0; kk < BK / 16; ++kk) {
                                     const uint64_t adv = (uint64_t)(kk * 2);
-                                    if (leader) umma_f16(d_tmem, a_lo + adv, w_hi + adv, idescf, (j | kk) != 0);
-                                    if (leader) umma_f16(d_tmem, a_hi + adv, w_lo + adv, idescf, 1);
+                                    umma_f16(d_tmem, a_lo + adv, w_hi + adv, idescf, (j | kk) != 0);
+                                    umma_f16(d_tmem, a_hi + adv, w_lo + adv, idescf, 1);
                                 }
 #pragma unroll
                                 for (int kk = 0; kk < BK / 16; ++kk) {
                                     const uint64_t adv = (uint64_t)(kk * 2);
-                                    if (leader) umma_f16(d_tmem, a_hi + adv, w_hi + adv, idescf, 1);
+                                    umma_f16(d_tmem, a_hi + adv, w_hi + adv, idescf, 1);
                                 }
                                 release(s);
                                 if (++s == STEP_G2_STAGES) s = 0;
                             }
-                            if (leader) umma_commit(bar_tfull + 8 * acc);
+                            umma_commit(bar_tfull + 8 * acc);
                         }
                     }
                 }
@@ -814,19 +743,16 @@ rq_coupling_step_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __gr
     if (warp == 1) tmem_dealloc(tmem_base, 512);
 }
 
-template <int NB, bool TAILS, int EWG>
+// Four epilogue warpgroups where a column tile has at least four features, else two (only NB = 16 without tails).
+template <int NB, bool TAILS>
 static int launch_step(const NfkCouplingStep* d, StepParams& p, cudaStream_t st) {
+    constexpr int EWG = StepCfg<NB, TAILS, 2>::TF >= 4 ? 4 : 2;
     using Cfg = StepCfg<NB, TAILS, EWG>;
-    static int cluster_pref = 0;
-    if (!cluster_pref) {
-        const char* e = getenv("NFK_CLUSTER");
-        cluster_pref = (e && e[0] == '1') ? 1 : 2;
-    }
     const int H = p.H;
     const int nch = H > 128 ? 2 : 1, ch = H / nch;
     // trunk-only launches run single CTAs: their TMA stores read R while a cluster peer could already multicast the next
     // tile's weights over it
-    const int CL = (cluster_pref == 2 && !p.trunk_only && p.num_m_tiles >= 2 && ch % 16 == 0 && (ch / 2) % 8 == 0) ? 2 : 1;
+    const int CL = (!p.trunk_only && p.num_m_tiles >= 2 && ch % 16 == 0 && (ch / 2) % 8 == 0) ? 2 : 1;
     const int L = p.num_layers - 1;
     CUtensorMap ma_hi, ma_lo, mw0_hi, mw0_lo, mwt_hi, mwt_lo, mwf_hi, mwf_lo;
     int rc;
@@ -846,20 +772,13 @@ static int launch_step(const NfkCouplingStep* d, StepParams& p, cudaStream_t st)
         if ((rc = make_map(&mh_lo, (const __half*)d->h_lo, p.n_rows, H, d->ldh, BM))) return rc;
     } else {
         const int packed_rows = p.d_t * Cfg::MP;
-        { const char* e = getenv("NFK_STEP_X_PREFETCH"); p.x_prefetch = (e && e[0] == '1') ? 1 : 0; }
-        { const char* e = getenv("NFK_STEP_K16"); p.k16 = (e && e[0] == '1') ? 1 : 0; }      // measured slower (168.7 vs 155.2 ms per step): off
-        if (p.k16) {
-            if ((rc = make_map_k16(&mwf_hi, (const __half*)d->wp_hi, packed_rows, H, d->ldwp, Cfg::BN / CL))) return rc;
-            if ((rc = make_map_k16(&mwf_lo, (const __half*)d->wp_lo, packed_rows, H, d->ldwp, Cfg::BN / CL))) return rc;
-        } else {
-            if ((rc = make_map(&mwf_hi, (const __half*)d->wp_hi, packed_rows, H, d->ldwp, Cfg::BN / CL))) return rc;
-            if ((rc = make_map(&mwf_lo, (const __half*)d->wp_lo, packed_rows, H, d->ldwp, Cfg::BN / CL))) return rc;
-        }
+        if ((rc = make_map(&mwf_hi, (const __half*)d->wp_hi, packed_rows, H, d->ldwp, Cfg::BN / CL))) return rc;
+        if ((rc = make_map(&mwf_lo, (const __half*)d->wp_lo, packed_rows, H, d->ldwp, Cfg::BN / CL))) return rc;
         p.num_n_tiles = (p.d_t + Cfg::TF - 1) / Cfg::TF;
         p.tma_y = (p.y && !p.t_cols && p.t_col0 % 4 == 0 && p.ldy % 4 == 0 && aligned16(p.y)) ? 1 : 0;
         // inputs as TMA boxes of TF columns: consecutive columns from a 16-byte aligned first column (tiles start at multiples of TF >= 4 floats...
         // TF = 2: 8-byte boxes are below the TMA minimum -> cp.async staging)
-        p.tma_x = (!p.t_cols && Cfg::TF >= 4 && p.t_col0 % 4 == 0 && p.ldx % 4 == 0 && aligned16(p.x) && !getenv("NFK_STEP_NO_TMA_X")) ? 1 : 0;
+        p.tma_x = (!p.t_cols && Cfg::TF >= 4 && p.t_col0 % 4 == 0 && p.ldx % 4 == 0 && aligned16(p.x)) ? 1 : 0;
         if (p.tma_x && (rc = make_out_map(&mx, const_cast<float*>(p.x), p.n_rows, p.t_col0 + p.d_t, p.ldx, Cfg::TF, BM))) return rc;
         if (p.tma_y && (rc = make_out_map(&my, p.y, p.n_rows, p.t_col0 + p.d_t, p.ldy, Cfg::YROW, BM))) return rc;
         if (p.pair_only) {
@@ -901,16 +820,6 @@ static int launch_step(const NfkCouplingStep* d, StepParams& p, cudaStream_t st)
     return check_launch("rq_coupling_step_kernel");
 }
 
-// epilogue warpgroups: NFK_STEP_EWG=2 selects the two-warpgroup variant (A/B measurements), default four
-static int step_ewg() {
-    static int v = 0;
-    if (!v) {
-        const char* e = getenv("NFK_STEP_EWG");
-        v = (e && e[0] == '2') ? 2 : 4;
-    }
-    return v;
-}
-
 }  // namespace tc
 }  // namespace nfk
 
@@ -947,19 +856,6 @@ extern "C" int nfk_rq_coupling_step_f16x3(const NfkCouplingStep* d, void* stream
     NFK_REQUIRE(d->n_rows < (1ll << 31), "n_rows too large for one launch");
     tc::StepParams p;
     memset(&p, 0, sizeof(p));
-    p.drain_f = tc::STEP_DRAIN_FINAL_DEFAULT;
-    {
-        static int mma_pref = 0, drain_t_pref = 0;
-        if (!mma_pref) {
-            const char* e = getenv("NFK_STEP_MMA_WARPS");
-            mma_pref = (e && e[0] == '2') ? 2 : 1;
-            const char* t = getenv("NFK_STEP_TRUNK_DRAIN");
-            drain_t_pref = t ? atoi(t) : tc::STEP_DRAIN_TRUNK_DEFAULT;
-            if (drain_t_pref < 1) drain_t_pref = tc::STEP_DRAIN_TRUNK_DEFAULT;
-        }
-        p.mma_warps = mma_pref;
-        p.drain_t = drain_t_pref;
-    }
     p.bias_trunk = d->bias_trunk; p.skip_buf = (float4*)d->workspace; p.H = d->hidden_features; p.K0 = d->in_features;
     p.num_layers = 1 + d->num_square_layers; p.act_scale = ldexpf(1.0f, d->act_exp); p.trunk_only = trunk_only ? 1 : 0;
     for (int l = 0; l < p.num_layers; ++l) {
@@ -976,7 +872,7 @@ extern "C" int nfk_rq_coupling_step_f16x3(const NfkCouplingStep* d, void* stream
     cudaStream_t st = (cudaStream_t)stream;
     if (trunk_only) {
         NFK_REQUIRE(d->h_lo && d->ldh % 8 == 0 && aligned16(d->h_hi) && aligned16(d->h_lo), "bad trunk output pair");
-        return tc::step_ewg() == 4 ? tc::launch_step<8, true, 4>(d, p, st) : tc::launch_step<8, true, 2>(d, p, st);
+        return tc::launch_step<8, true>(d, p, st);               // four epilogue warpgroups
     }
     int rc = make_spline_params(d->spline, &p.sp);
     if (rc) return rc;
@@ -990,27 +886,12 @@ extern "C" int nfk_rq_coupling_step_f16x3(const NfkCouplingStep* d, void* stream
     p.ldx = d->ldx; p.ldy = d->ldy; p.d_t = d->d_t; p.inverse = d->inverse;
     p.inv_acc_scale_f = ldexpf(1.0f, -(d->act_exp + d->wp_exp));
     p.pair_only = d->y_hi ? 1 : 0; p.out_scale = ldexpf(1.0f, d->y_exp);
-    {
-        static int drain_pref = 0;
-        if (!drain_pref) {
-            const char* e = getenv("NFK_STEP_DRAIN");
-            drain_pref = e ? atoi(e) : tc::STEP_DRAIN_FINAL_DEFAULT;
-            if (drain_pref < 1) drain_pref = tc::STEP_DRAIN_FINAL_DEFAULT;
-        }
-        p.drain_f = drain_pref;
-    }
     const bool tails = d->spline->linear_tails != 0;
-    // four epilogue warpgroups where a column tile has at least four features, else two
-#define NFK_STEP(NB)                                                                                                       \
-    if (tc::step_ewg() == 4 && tc::StepCfg<NB, true, 2>::TF >= 4 && tails) return tc::launch_step<NB, true, tc::StepCfg<NB, true, 2>::TF >= 4 ? 4 : 2>(d, p, st);     \
-    if (tc::step_ewg() == 4 && tc::StepCfg<NB, false, 2>::TF >= 4 && !tails) return tc::launch_step<NB, false, tc::StepCfg<NB, false, 2>::TF >= 4 ? 4 : 2>(d, p, st);  \
-    return tails ? tc::launch_step<NB, true, 2>(d, p, st) : tc::launch_step<NB, false, 2>(d, p, st)
     switch (d->spline->num_bins) {
-        case 4: NFK_STEP(4);
-        case 8: NFK_STEP(8);
-        case 10: NFK_STEP(10);
-        case 16: NFK_STEP(16);
+        case 4: return tails ? tc::launch_step<4, true>(d, p, st) : tc::launch_step<4, false>(d, p, st);
+        case 8: return tails ? tc::launch_step<8, true>(d, p, st) : tc::launch_step<8, false>(d, p, st);
+        case 10: return tails ? tc::launch_step<10, true>(d, p, st) : tc::launch_step<10, false>(d, p, st);
+        case 16: return tails ? tc::launch_step<16, true>(d, p, st) : tc::launch_step<16, false>(d, p, st);
     }
-#undef NFK_STEP
     return fail(NFK_E_UNSUPPORTED, "num_bins=%d has no coupling-step kernel instance", d->spline->num_bins);
 }

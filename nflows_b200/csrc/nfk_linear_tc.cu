@@ -38,8 +38,6 @@
 //         load in flight, the tensor pipe waited a full HBM round trip per pair -- ncu r2: 21 % tensor, 39 % DRAM, 31 % L2);
 //         + 8 warps x 2 x 4 KB store staging;
 //   TMEM: 2 partial accumulators x 256 columns.
-#include <stdlib.h>
-
 #include <mutex>
 
 #include "tc_common.cuh"
@@ -68,8 +66,6 @@ struct Params {
     int tma_store;           // outputs are TMA-addressable (16-byte aligned bases and row pitches): staged stores
     int y_first_col;         // the fp32 result is only needed for columns >= y_first_col (32-column chunks below it are skipped)
     int a_stages, w_stages;  // ring depths
-    int mma_warps;           // 2: two MMA-issuing warps take alternate partial sums
-    int drain;               // K-slabs accumulated in TMEM per partial sum (DRAIN_SLABS_LINEAR by default)
     int w_slot_bytes;        // bytes per W ring slot (hi part first, lo part at w_slot_bytes / 2)
     // affine-coupling epilogue (nfk_affine_coupling_final_f16x3): the GEMM result is the conditioner's parameter row --
     // interleaved (shift_j, raw scale_j) pairs when c_mult == 2, shift_j when 1 -- consumed in registers, never stored
@@ -79,7 +75,6 @@ struct Params {
     float* c_lad;            // running log|det| per row (atomicAdd of this thread's share), may be NULL
     int64_t ldcx, ldcy;
     int c_col0, c_dt, c_mult, c_act, c_inverse;
-    long long* prof;         // NFK_LINEAR_PROF=<device address>: per-CTA cycle counters [8] (scripts/linear_prof.py), else NULL
 };
 
 // Operand rings share LIN_RING_BYTES: LIN_W_STAGES weight slots of [W hi | W lo] sized for the launch's column tile (BN rows of
@@ -122,13 +117,7 @@ __device__ __forceinline__ bool tile_of(const int it, const int n_inner, const i
     return t < units * num_n;
 }
 
-// PAIR (with CL = 2): the two CTAs of a cluster form a tcgen05 CTA PAIR (cta_group::2).  ONE 256 x BN x 16 MMA, issued by the
-// leader (cluster rank 0), drives both SMs' tensor cores: each CTA supplies its own 128 A rows and HALF of the weight tile from
-// its own shared memory.  Per SM that halves the weight bytes written by TMA and read by the MMA -- the multicast form moves
-// A + the FULL weight tile through every SM's 128 B/clk shared-memory port (ncu r2: 43 % tensor pipe at ~100 B/clk of operand
-// traffic).  Every TMA load of either CTA counts its bytes on the LEADER's "full" barrier; the leader's tcgen05.commit releases
-// ring slots and accumulators in both CTAs; the epilogue warps of both CTAs report drained accumulators to the leader.
-template <int CL, bool PAIR>
+template <int CL>
 __global__ void __launch_bounds__(THREADS, 1)
 linear_f16x3_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_constant__ CUtensorMap map_a_lo,
                      const __grid_constant__ CUtensorMap map_w_hi, const __grid_constant__ CUtensorMap map_w_lo,
@@ -139,7 +128,6 @@ linear_f16x3_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_c
     extern __shared__ uint8_t smem_raw[];
     const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;      // SWIZZLE_128B needs 1024-byte alignment
     uint8_t* smem_gen = smem_raw + (smem_base - smem_u32(smem_raw));
-    static_assert(!PAIR || CL == 2, "a CTA pair is a cluster of two");
     const int LIN_A_STAGES = p.a_stages, LIN_W_STAGES = p.w_stages;
     const uint32_t LIN_W_STAGE_BYTES = (uint32_t)p.w_slot_bytes, W_LO = LIN_W_STAGE_BYTES / 2;
     const uint32_t ring_w = smem_base + LIN_A_STAGES * LIN_A_STAGE_BYTES;
@@ -154,21 +142,20 @@ linear_f16x3_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_c
 
     if (threadIdx.x == 0) {
         for (int s = 0; s < LIN_A_STAGES; ++s) { mbar_init(bar_afull + 8 * s, 1); mbar_init(bar_aempty + 8 * s, 1); }
-        // multicast form: both CTAs' MMA threads release a weight slot (the peer multicasts into it); pair form: the leader's
-        // commit reaches both CTAs' barriers
-        for (int s = 0; s < LIN_W_STAGES; ++s) { mbar_init(bar_wfull + 8 * s, 1); mbar_init(bar_wempty + 8 * s, PAIR ? 1 : CL); }
-        for (int a = 0; a < 2; ++a) { mbar_init(bar_tfull + 8 * a, 1); mbar_init(bar_tempty + 8 * a, PAIR ? 16 : 8); }
+        // both CTAs' MMA threads of a cluster release a weight slot (the peer multicasts into it)
+        for (int s = 0; s < LIN_W_STAGES; ++s) { mbar_init(bar_wfull + 8 * s, 1); mbar_init(bar_wempty + 8 * s, CL); }
+        for (int a = 0; a < 2; ++a) { mbar_init(bar_tfull + 8 * a, 1); mbar_init(bar_tempty + 8 * a, 8); }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
         prefetch_tmap(&map_a_hi); prefetch_tmap(&map_a_lo); prefetch_tmap(&map_w_hi); prefetch_tmap(&map_w_lo);
     }
-    if (warp == 1) { if (PAIR) tmem_alloc_pair(smem_u32(tmem_slot), 512); else tmem_alloc(smem_u32(tmem_slot), 512); }
+    if (warp == 1) tmem_alloc(smem_u32(tmem_slot), 512);
     tc_fence_before();
     if (CL > 1) cluster_sync_all(); else __syncthreads();
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
     const int cta_rank = CL > 1 ? (int)cluster_ctarank() : 0;
     constexpr uint16_t cl_mask = (uint16_t)((1u << CL) - 1);
-    const int num_groups = (num_k + p.drain - 1) / p.drain;               // partial sums per tile
+    const int num_groups = (num_k + DRAIN_SLABS_LINEAR - 1) / DRAIN_SLABS_LINEAR;   // partial sums per tile
 
     if (warp < 4) {
     asm volatile("setmaxnreg.dec.sync.aligned.u32 40;" ::: "memory");     // hand registers to the epilogue warpgroups
@@ -184,16 +171,9 @@ linear_f16x3_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_c
                     mbar_wait(bar_aempty + 8 * stage, phase ^ 1);
                     const uint32_t full = bar_afull + 8 * stage;
                     const uint32_t sa = smem_base + stage * LIN_A_STAGE_BYTES;
-                    if (PAIR) {                                            // both CTAs' rows are counted on the leader's barrier
-                        const uint32_t lead = mapa_rank(full, 0);
-                        if (cta_rank == 0) mbar_expect_tx(full, 4u * A_BYTES);
-                        tma_load_2d_pair(sa, &map_a_hi, lead, ks * BK, m0);
-                        tma_load_2d_pair(sa + A_BYTES, &map_a_lo, lead, ks * BK, m0);
-                    } else {
-                        mbar_expect_tx(full, 2u * A_BYTES);
-                        tma_load_2d(sa, &map_a_hi, full, ks * BK, m0);
-                        tma_load_2d(sa + A_BYTES, &map_a_lo, full, ks * BK, m0);
-                    }
+                    mbar_expect_tx(full, 2u * A_BYTES);
+                    tma_load_2d(sa, &map_a_hi, full, ks * BK, m0);
+                    tma_load_2d(sa + A_BYTES, &map_a_lo, full, ks * BK, m0);
                     if (++stage == LIN_A_STAGES) { stage = 0; phase ^= 1; }
                 }
             }
@@ -212,14 +192,6 @@ linear_f16x3_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_c
                     mbar_wait(bar_wempty + 8 * stage, phase ^ 1);          // every CTA of the cluster has released the slot
                     const uint32_t full = bar_wfull + 8 * stage;
                     const uint32_t sw = ring_w + stage * LIN_W_STAGE_BYTES;
-                    if (PAIR) {                  // this CTA's half of the tile's weight rows, at the slot base of its own shared memory
-                        const uint32_t lead = mapa_rank(full, 0);
-                        if (cta_rank == 0) mbar_expect_tx(full, tx_bytes);
-                        tma_load_2d_pair(sw, &map_w_hi, lead, ks * BK, n0 + cta_rank * wrows);
-                        tma_load_2d_pair(sw + W_LO, &map_w_lo, lead, ks * BK, n0 + cta_rank * wrows);
-                        if (++stage == LIN_W_STAGES) { stage = 0; phase ^= 1; }
-                        continue;
-                    }
                     mbar_expect_tx(full, tx_bytes);
                     if (CL == 1) {
                         tma_load_2d(sw, &map_w_hi, full, ks * BK, n0);
@@ -233,50 +205,27 @@ linear_f16x3_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_c
                 }
             }
         }
-    } else if ((warp == 1 || (warp == 3 && p.mma_warps == 2)) && (!PAIR || cta_rank == 0)) {
-        // ================================================= MMA issuers: one ELECTED thread per issuing warp (uniform datapath:
-        // descriptors in uniform registers, tcgen05.mma back to back -- see tc_common.cuh: elect_one).
+    } else if (warp == 1) {
+        // ================================================= MMA issuer: one ELECTED thread (uniform datapath: descriptors in
+        // uniform registers, tcgen05.mma back to back -- see tc_common.cuh: elect_one).
         // Per K-slab: the two small cross terms (a_lo w_hi, a_hi w_lo), then the main product, then both ring slots are released;
-        // a partial sum (one TMEM buffer) covers DRAIN_SLABS_LINEAR slabs.  TWO issuing warps take alternate partial sums (warp 1:
-        // buffer 0, warp 3: buffer 1): every tcgen05.mma costs the issuing thread ~190 cycles of ELECT / R2UR operand moves
-        // against ~100 cycles of tensor work, so one issuer left the tensor pipe half idle (ncu r2).
+        // a partial sum (one TMEM buffer, alternating) covers DRAIN_SLABS_LINEAR slabs.
         if (elect_one()) {
-            const bool leader = true;
-            const int my = warp == 1 ? 0 : 1;
-            const bool solo = p.mma_warps != 2;
-            const uint32_t idesc = make_idesc(p.BN, PAIR ? 2 * BM : BM);
-            auto mma = [&](uint32_t d, uint64_t a, uint64_t b, uint32_t accumulate) {
-                if (!leader) return;
-                if (PAIR) umma_f16_pair(d, a, b, idesc, accumulate); else umma_f16(d, a, b, idesc, accumulate);
-            };
+            const uint32_t idesc = make_idesc(p.BN);
             int sa_i = 0; uint32_t pa = 0;
             int sw_i = 0; uint32_t pw = 0;
             uint32_t gc = 0;                                              // partial sums so far: buffer gc & 1, use gc >> 1 of it
             int tm, tn;
-            long long t_tempty = 0, t_full = 0;
-            const long long t_begin = p.prof ? clock64() : 0;
             for (int it = 0; tile_of<CL>(it, p.n_inner, p.num_m_tiles, p.num_n_tiles, cta_rank, tm, tn); ++it) {
                 for (int g = 0; g < num_groups; ++g, ++gc) {
-                    const int slabs = min(p.drain, num_k - g * p.drain);
-                    if (!solo && (int)(gc & 1u) != my) {                  // the other issuer's partial sum: step over its slots
-                        for (int j = 0; j < slabs; ++j) {
-                            if (++sa_i == LIN_A_STAGES) { sa_i = 0; pa ^= 1; }
-                            if (++sw_i == LIN_W_STAGES) { sw_i = 0; pw ^= 1; }
-                        }
-                        continue;
-                    }
+                    const int slabs = min(DRAIN_SLABS_LINEAR, num_k - g * DRAIN_SLABS_LINEAR);
                     const int acc = gc & 1u;
                     const uint32_t acc_phase = (gc >> 1) & 1u;
-                    long long t0 = p.prof ? clock64() : 0;
-                    if (PAIR) mbar_wait_cluster(bar_tempty + 8 * acc, acc_phase ^ 1);   // both CTAs' epilogues have drained it
-                    else mbar_wait(bar_tempty + 8 * acc, acc_phase ^ 1);  // epilogue has drained this partial accumulator
-                    if (p.prof) t_tempty += clock64() - t0;
+                    mbar_wait(bar_tempty + 8 * acc, acc_phase ^ 1);       // epilogue has drained this partial accumulator
                     const uint32_t d_tmem = tmem_base + acc * BN_MAX;
                     for (int j = 0; j < slabs; ++j) {
-                        if (p.prof) t0 = clock64();
                         mbar_wait(bar_afull + 8 * sa_i, pa);               // TMA bytes have landed
                         mbar_wait(bar_wfull + 8 * sw_i, pw);
-                        if (p.prof) t_full += clock64() - t0;
                         tc_fence_after();
                         const uint32_t sa = smem_base + sa_i * LIN_A_STAGE_BYTES;
                         const uint32_t sw = ring_w + sw_i * LIN_W_STAGE_BYTES;
@@ -285,35 +234,22 @@ linear_f16x3_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_c
 #pragma unroll
                         for (int kk = 0; kk < BK / 16; ++kk) {             // UMMA K = 16 fp16 = 32 bytes = +2 in descriptor units
                             const uint64_t adv = (uint64_t)(kk * 2);
-                            mma(d_tmem, a_lo + adv, w_hi + adv, (j | kk) != 0);
-                            mma(d_tmem, a_hi + adv, w_lo + adv, 1);
+                            umma_f16(d_tmem, a_lo + adv, w_hi + adv, idesc, (j | kk) != 0);
+                            umma_f16(d_tmem, a_hi + adv, w_lo + adv, idesc, 1);
                         }
 #pragma unroll
                         for (int kk = 0; kk < BK / 16; ++kk) {
                             const uint64_t adv = (uint64_t)(kk * 2);
-                            mma(d_tmem, a_hi + adv, w_hi + adv, 1);
+                            umma_f16(d_tmem, a_hi + adv, w_hi + adv, idesc, 1);
                         }
-                        if (leader) {
-                            if (PAIR) {                                                     // both CTAs' slots, when the MMAs retire
-                                umma_commit_pair(bar_aempty + 8 * sa_i, cl_mask);
-                                umma_commit_pair(bar_wempty + 8 * sw_i, cl_mask);
-                            } else {
-                                umma_commit(bar_aempty + 8 * sa_i);                         // frees the slots when the MMAs retire
-                                if (CL == 1) umma_commit(bar_wempty + 8 * sw_i);
-                                else umma_commit_multicast(bar_wempty + 8 * sw_i, cl_mask);   // ... the weight slot in every CTA of the cluster
-                            }
-                        }
+                        umma_commit(bar_aempty + 8 * sa_i);                             // frees the slots when the MMAs retire
+                        if (CL == 1) umma_commit(bar_wempty + 8 * sw_i);
+                        else umma_commit_multicast(bar_wempty + 8 * sw_i, cl_mask);     // ... the weight slot in every CTA of the cluster
                         if (++sa_i == LIN_A_STAGES) { sa_i = 0; pa ^= 1; }
                         if (++sw_i == LIN_W_STAGES) { sw_i = 0; pw ^= 1; }
                     }
-                    if (leader) {                                                       // partial sum complete -> drain
-                        if (PAIR) umma_commit_pair(bar_tfull + 8 * acc, cl_mask); else umma_commit(bar_tfull + 8 * acc);
-                    }
+                    umma_commit(bar_tfull + 8 * acc);                      // partial sum complete -> drain
                 }
-            }
-            if (p.prof && warp == 1) {
-                long long* o = p.prof + (size_t)blockIdx.x * 16;
-                o[0] = clock64() - t_begin; o[1] = t_tempty; o[2] = t_full;
             }
         }
     }
@@ -333,8 +269,6 @@ linear_f16x3_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_c
         const uint32_t stg_u32 = smem_base + LIN_STG_OFF + (warp - 4) * 2 * LIN_STG_BYTES;
         int stg_buf = 0;
         int tm, tn;
-        long long t_tfull = 0, t_out = 0, t_pro = 0, t_drain = 0, t_bias = 0, t_wait = 0, t_y = 0, t_pair = 0;
-        const long long e_begin = p.prof ? clock64() : 0;
         // this lane's float4 of the bias of tile `it` (zeros past the tile / the matrix, or without a bias)
         auto bias_of = [&](int it) -> float4 {
             float4 b = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -356,7 +290,6 @@ linear_f16x3_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_c
         };
         float4 bias_cur = bias_of(0);
         for (int it = 0; tile_of<CL>(it, p.n_inner, p.num_m_tiles, p.num_n_tiles, cta_rank, tm, tn); ++it) {
-            long long e0 = p.prof ? clock64() : 0;
             const int64_t row = (int64_t)tm * BM + q * 32 + lane;
             const int n0 = tn * p.BN + half * HALF;
             // The running sums start from bias (+ residual when no relu sits between them): the loads are issued here, at the
@@ -377,12 +310,11 @@ linear_f16x3_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_c
                 }
             }
             float sum[HALF];
-            const long long b0 = p.prof ? clock64() : 0;
             // The running sums live in the accumulators' power-of-two scaled domain (exact) and start from the bias: ONE coalesced
             // float4 per thread (lane l: columns 4l..4l+3 of this warp's column half; fetched during the PREVIOUS tile, see
             // bias_of) broadcast by shuffles.  The first form -- 32 broadcast float4 loads, each followed by its adds -- serialised
             // 32 L2 latencies per tile: 8 600 of a tile's 28 000 cycles, the MMA thread waiting for drained accumulators meanwhile
-            // (r2 cycle counters, scripts/linear_prof.py; L1 keeps little beside 227 KB of shared memory).
+            // (r2 cycle counters, profiles/linear_cycles_r2.txt; L1 keeps little beside 227 KB of shared memory).
             const float4 mine = make_float4(bias_cur.x * p.acc_scale, bias_cur.y * p.acc_scale, bias_cur.z * p.acc_scale,
                                             bias_cur.w * p.acc_scale);
             if (fold_residual) {
@@ -421,11 +353,8 @@ linear_f16x3_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_c
                     sum[c + 3] = __shfl_sync(0xffffffffu, mine.w, c >> 2);
                 }
             }
-            if (p.prof) t_bias += clock64() - b0;
-            if (p.prof) { const long long n = clock64(); t_pro += n - e0; e0 = n; }
             for (int g = 0; g < num_groups; ++g) {
                 mbar_wait(bar_tfull + 8 * acc, acc_phase);
-                if (p.prof) { const long long n = clock64(); t_tfull += n - e0; e0 = n; }
                 tc_fence_after();
                 const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + acc * BN_MAX + half * HALF;
 #pragma unroll
@@ -447,12 +376,8 @@ linear_f16x3_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_c
                 }
                 tc_fence_before();
                 __syncwarp();
-                if (lane == 0) {
-                    if (PAIR) mbar_arrive_cluster(mapa_rank(bar_tempty + 8 * acc, 0));   // the leader's MMA thread reuses the accumulator
-                    else mbar_arrive(bar_tempty + 8 * acc);
-                }
+                if (lane == 0) mbar_arrive(bar_tempty + 8 * acc);
                 if (++acc == 2) { acc = 0; acc_phase ^= 1; }
-                if (p.prof) { const long long n = clock64(); t_drain += n - e0; e0 = n; }
             }
             const float4 bias_nxt = bias_of(it + 1);      // lands while this tile is written out
             if (p.tma_store) {
@@ -484,10 +409,8 @@ linear_f16x3_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_c
                 // beyond the tensor, so ragged tiles need no guards
                 const int row0 = tm * BM + q * 32;
                 auto stage_begin = [&]() -> uint4* {
-                    const long long w0 = p.prof ? clock64() : 0;
                     if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");   // the chunk before last has left
                     __syncwarp();
-                    if (p.prof) t_wait += clock64() - w0;
                     return reinterpret_cast<uint4*>(stg_gen + stg_buf * LIN_STG_BYTES) + lane * 8;
                 };
                 auto stage_end = [&](const CUtensorMap* map, int c0) {
@@ -496,7 +419,6 @@ linear_f16x3_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_c
                     if (lane == 0) tma_store_2d(map, stg_u32 + stg_buf * LIN_STG_BYTES, c0, row0);
                     stg_buf ^= 1;
                 };
-                const long long y0 = p.prof ? clock64() : 0;
                 if (p.y) {
 #pragma unroll
                     for (int ch = 0; ch < HALF / 32; ++ch) {
@@ -525,8 +447,6 @@ linear_f16x3_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_c
                         stage_end(&map_y, col0);
                     }
                 }
-                const long long y1 = p.prof ? clock64() : 0;
-                if (p.prof) t_y += y1 - y0;
                 if (p.y_hi) {
 #pragma unroll
                     for (int ch = 0; ch < HALF / 64; ++ch) {
@@ -559,10 +479,8 @@ linear_f16x3_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_c
                             vh[j] = *reinterpret_cast<const uint4*>(h2);
                             vl[j] = *reinterpret_cast<const uint4*>(l2);
                         }
-                        const long long w0 = p.prof ? clock64() : 0;
                         if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
                         __syncwarp();
-                        if (p.prof) t_wait += clock64() - w0;
 #pragma unroll
                         for (int j = 0; j < 8; ++j) {
                             if (j < pieces) {
@@ -581,7 +499,6 @@ linear_f16x3_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_c
                         stg_buf = 0;
                     }
                 }
-                if (p.prof) t_pair += clock64() - y1;
             } else if (p.cx) {
                 // ---- affine / additive coupling (coupling.py:212-269 of the reference) on the parameters held in registers:
                 // y_j = x_j * s_j + t_j (inverse: (x_j - t_j) / s_j), log|det| += +-sum_j log s_j
@@ -678,12 +595,6 @@ linear_f16x3_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_c
             }
             __syncwarp();
             bias_cur = bias_nxt;
-            if (p.prof) t_out += clock64() - e0;
-        }
-        if (p.prof && warp == 4 && lane == 0) {
-            long long* o = p.prof + (size_t)blockIdx.x * 16;
-            o[3] = clock64() - e_begin; o[4] = t_tfull; o[5] = t_drain; o[6] = t_out; o[7] = t_pro;
-            o[8] = t_bias; o[9] = t_wait; o[10] = t_y; o[11] = t_pair;
         }
         if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");   // staging must outlive its stores
         if (flag && p.flags) atomicOr(p.flags, flag);
@@ -691,7 +602,7 @@ linear_f16x3_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_c
 
     tc_fence_before();
     if (CL > 1) cluster_sync_all(); else __syncthreads();   // no CTA exits while a peer may still signal its barriers
-    if (warp == 1) { if (PAIR) tmem_dealloc_pair(tmem_base, 512); else tmem_dealloc(tmem_base, 512); }
+    if (warp == 1) tmem_dealloc(tmem_base, 512);
 }
 
 // ---------------------------------------------------------------- fp32 -> fp16 (hi, lo) split pair, optional relu
@@ -831,21 +742,6 @@ int make_map(CUtensorMap* map, const __half* base, int64_t rows, int K, int64_t 
     return NFK_OK;
 }
 
-// K-major operand tile of 16 halfs (one UMMA K step) per row: 32-byte rows, SWIZZLE_32B (the coupling-step kernel's final layer)
-int make_map_k16(CUtensorMap* map, const __half* base, int64_t rows, int K, int64_t ld, int box_rows) {
-    EncodeTiledFn fn = encode_fn();
-    if (!fn) return fail(NFK_E_CUDA, "cuTensorMapEncodeTiled is not available from the driver");
-    cuuint64_t dims[2] = {(cuuint64_t)K, (cuuint64_t)rows};
-    cuuint64_t strides[1] = {(cuuint64_t)ld * 2};
-    cuuint32_t box[2] = {16u, (cuuint32_t)box_rows};
-    cuuint32_t estr[2] = {1, 1};
-    CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<__half*>(base), dims, strides, box, estr,
-                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_32B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(NFK_E_CUDA, "cuTensorMapEncodeTiled (k16) failed with CUresult %d", (int)r);
-    return NFK_OK;
-}
-
 int sm_count() {
     static std::atomic<int> counts[64];                      // per device
     int dev = 0;
@@ -865,13 +761,6 @@ int sm_count() {
 using namespace nfk;
 
 static bool pow2_exp_ok(int e) { return e >= -60 && e <= 60; }
-static int max_clusters_hint(int cl) { return nfk::tc::sm_count() / cl; }
-// bytes of one half (hi or lo) of a weight slot for the column tile the launch will use: BN rows x 64 bytes
-static int bn_rows_bytes(int out_features) {
-    int tiles = (out_features + nfk::tc::BN_MAX - 1) / nfk::tc::BN_MAX;
-    int bn = ((out_features + tiles - 1) / tiles + 15) / 16 * 16;
-    return bn * nfk::tc::ROW_BYTES;
-}
 
 extern "C" int nfk_split_f16(const float* x, int64_t ldx, int32_t n_cols, int relu, int32_t scale_exp, void* hi, void* lo,
                              int64_t ldo, int64_t n_rows, int32_t* flags, void* stream) {
@@ -967,24 +856,11 @@ static int linear_f16x3_launch(const void* a_hi_, const void* a_lo_, int64_t lda
     p.ldr = ldr; p.ldy = ldy; p.lds = lds; p.n_rows = n_rows; p.K = in_features; p.N = out_features;
     p.relu_out = relu_out; p.split_relu = split_relu;
     p.y_first_col = y_first_col > 0 ? y_first_col : 0;
-    { const char* e = getenv("NFK_LINEAR_PROF"); p.prof = e ? reinterpret_cast<long long*>(strtoull(e, nullptr, 0)) : nullptr; }
     p.cx = nullptr; p.cy = nullptr; p.c_cols = nullptr; p.c_lad = nullptr; p.ldcx = p.ldcy = 0;
     p.c_col0 = p.c_dt = p.c_mult = p.c_act = p.c_inverse = 0;
     if (ce) {
         p.cx = ce->x; p.cy = ce->y; p.c_cols = ce->t_cols; p.c_lad = ce->lad; p.ldcx = ce->ldx; p.ldcy = ce->ldy;
         p.c_col0 = ce->t_col0; p.c_dt = ce->d_t; p.c_mult = ce->mult; p.c_act = ce->act; p.c_inverse = ce->inverse;
-    }
-    {
-        static int mma_pref = 0, drain_pref = 0;
-        if (!mma_pref) {
-            const char* e = getenv("NFK_LINEAR_MMA_WARPS");
-            mma_pref = (e && e[0] == '2') ? 2 : 1;
-            const char* d = getenv("NFK_LINEAR_DRAIN");
-            drain_pref = d ? atoi(d) : tc::DRAIN_SLABS_LINEAR;
-            if (drain_pref < 1) drain_pref = tc::DRAIN_SLABS_LINEAR;
-        }
-        p.mma_warps = mma_pref;
-        p.drain = drain_pref;
     }
     p.num_n_tiles = (out_features + tc::BN_MAX - 1) / tc::BN_MAX;
     int bn = (out_features + p.num_n_tiles - 1) / p.num_n_tiles;
@@ -993,19 +869,11 @@ static int linear_f16x3_launch(const void* a_hi_, const void* a_lo_, int64_t lda
     p.num_n_tiles = (out_features + bn - 1) / bn;
     p.num_m_tiles = (int)((n_rows + tc::BM - 1) / tc::BM);
 
-    static int cluster_pref = 0;
-    if (!cluster_pref) {
-        const char* e = getenv("NFK_CLUSTER");
-        cluster_pref = (e && e[0] == '1') ? 1 : (e && e[0] == '3') ? 3 : 2;
-    }
-    const int CL = (cluster_pref >= 2 && p.num_m_tiles >= 2) ? 2 : 1;
-    // CTA pairs (cta_group::2): UMMA M = 256 needs N a multiple of 16 and each CTA's half a multiple of 8 rows
-    const bool pair = CL == 2 && cluster_pref == 3;
-    // ring split: weight slots hold this CTA's rows of a K-slab (all BN rows, or BN / 2 in a pair), hi part then lo part, each
-    // rounded to the 1024-byte swizzle alignment; the rest of the ring holds 16 KB A slots
-    const int w_rows = pair ? bn / 2 : bn;
-    p.w_slot_bytes = 2 * ((w_rows * tc::ROW_BYTES + 1023) / 1024 * 1024);
-    p.w_stages = pair ? 4 : 3;
+    const int CL = p.num_m_tiles >= 2 ? 2 : 1;
+    // ring split: weight slots hold the BN rows of a K-slab, hi part then lo part, each rounded to the 1024-byte swizzle
+    // alignment; the rest of the ring holds 16 KB A slots
+    p.w_slot_bytes = 2 * ((bn * tc::ROW_BYTES + 1023) / 1024 * 1024);
+    p.w_stages = 3;
     p.a_stages = (tc::LIN_RING_BYTES - p.w_stages * p.w_slot_bytes) / tc::LIN_A_STAGE_BYTES;
     if (p.a_stages > tc::LIN_A_STAGES_MAX) p.a_stages = tc::LIN_A_STAGES_MAX;
     CUtensorMap ma_hi, ma_lo, mw_hi, mw_lo;
@@ -1033,25 +901,18 @@ static int linear_f16x3_launch(const void* a_hi_, const void* a_lo_, int64_t lda
     static DeviceOnce attr_once;
     int attr_dev = 0;
     if (attr_once.pending(&attr_dev)) {
-        cudaError_t e = cudaFuncSetAttribute(tc::linear_f16x3_kernel<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::LIN_SMEM_BYTES);
+        cudaError_t e = cudaFuncSetAttribute(tc::linear_f16x3_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::LIN_SMEM_BYTES);
         if (e == cudaSuccess)
-            e = cudaFuncSetAttribute(tc::linear_f16x3_kernel<2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::LIN_SMEM_BYTES);
-        if (e == cudaSuccess)
-            e = cudaFuncSetAttribute(tc::linear_f16x3_kernel<2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::LIN_SMEM_BYTES);
+            e = cudaFuncSetAttribute(tc::linear_f16x3_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::LIN_SMEM_BYTES);
         if (e != cudaSuccess) return fail(NFK_E_CUDA, "cudaFuncSetAttribute(smem=%d): %s", tc::LIN_SMEM_BYTES, cudaGetErrorString(e));
         attr_once.mark(attr_dev);
     }
     const int units = (p.num_m_tiles + CL - 1) / CL;
+    const int max_clusters = tc::sm_count() / CL;
     // a CTA walks the column tiles of its row block back to back: the activations are read from HBM once and re-read from L2
     // (r1 measured no gain from this order -- its single 3-stage ring was bound by operand latency, not by DRAM traffic)
-    static int n_inner_pref = -1;
-    if (n_inner_pref < 0) {
-        const char* e = getenv("NFK_LINEAR_NINNER");
-        n_inner_pref = (e && e[0] == '0') ? 0 : 1;
-    }
-    p.n_inner = (n_inner_pref && p.num_n_tiles > 1 && units >= max_clusters_hint(CL)) ? 1 : 0;
+    p.n_inner = (p.num_n_tiles > 1 && units >= max_clusters) ? 1 : 0;
     const int work = units * p.num_n_tiles;
-    const int max_clusters = tc::sm_count() / CL;
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)(CL * (work < max_clusters ? work : max_clusters)));
     cfg.blockDim = dim3(tc::THREADS);
@@ -1062,9 +923,8 @@ static int linear_f16x3_launch(const void* a_hi_, const void* a_lo_, int64_t lda
     attr[0].val.clusterDim.x = CL; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    cudaError_t le = pair      ? cudaLaunchKernelEx(&cfg, tc::linear_f16x3_kernel<2, true>, ma_hi, ma_lo, mw_hi, mw_lo, my, myh, myl, myt, myht, mylt, p)
-                     : (CL == 2) ? cudaLaunchKernelEx(&cfg, tc::linear_f16x3_kernel<2, false>, ma_hi, ma_lo, mw_hi, mw_lo, my, myh, myl, myt, myht, mylt, p)
-                                 : cudaLaunchKernelEx(&cfg, tc::linear_f16x3_kernel<1, false>, ma_hi, ma_lo, mw_hi, mw_lo, my, myh, myl, myt, myht, mylt, p);
+    cudaError_t le = CL == 2 ? cudaLaunchKernelEx(&cfg, tc::linear_f16x3_kernel<2>, ma_hi, ma_lo, mw_hi, mw_lo, my, myh, myl, myt, myht, mylt, p)
+                             : cudaLaunchKernelEx(&cfg, tc::linear_f16x3_kernel<1>, ma_hi, ma_lo, mw_hi, mw_lo, my, myh, myl, myt, myht, mylt, p);
     if (le != cudaSuccess) return fail(NFK_E_CUDA, "cudaLaunchKernelEx(linear_f16x3_kernel, cluster %d): %s", CL, cudaGetErrorString(le));
     return check_launch("linear_f16x3_kernel");
 }

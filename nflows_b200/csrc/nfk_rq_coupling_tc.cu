@@ -11,8 +11,6 @@
 //     of its row in registers (K = 8 bins, linear tails: MP = 24, FPT = 5, BN = 240);
 //   * a CTA walks the N-tiles of one 128-row block consecutively, so every thread keeps the running log|det| of its row
 //     in a register and the row is finished (y written, lad_accum updated, deterministically) when the CTA moves on.
-#include <stdlib.h>
-
 #include "fused_spline.cuh"
 
 namespace nfk {
@@ -40,13 +38,10 @@ struct FusedParams {
     SplineParams sp;
 };
 
-// Epilogue warpgroups of the fused kernel (compile-time).  Measured on B200, cfg 3 (ms per step spent in this kernel):
+// Epilogue warpgroups of the fused kernel.  Measured on B200, cfg 3 (ms per step spent in this kernel):
 // EWG = 2 (5 features per thread, BN = 240, 40 N-tiles): 263;  EWG = 4 (2 features per thread, BN = 192, 49 N-tiles): 274 --
 // the epilogue is not what the tensor pipe waits for, and narrower tiles re-stream the activations more often.
-#ifndef NFK_FUSED_EWG
-#define NFK_FUSED_EWG 2
-#endif
-constexpr int EWG = NFK_FUSED_EWG;
+constexpr int EWG = 2;
 constexpr int FUSED_THREADS = 128 + 128 * EWG;
 // registers: the launch allocates floor(64K / threads) per thread; the control warpgroup shrinks to 40 and the epilogue
 // warpgroups share what that frees (setmaxnreg needs multiples of 8)
@@ -73,14 +68,11 @@ struct FusedCfg {
     static_assert(FPT >= 1 && BN <= BN_MAX, "unsupported bin count for the fused kernel");
 };
 
-// MODE 1: one CTA per 128-row block.
-// MODE 2: clusters of two CTAs on neighbouring 128-row blocks walking the same weight tiles in lockstep; each loads HALF of
-//         every weight slab and multicasts it into both CTAs' shared memory (halves the L2 -> SM weight stream; ncu: L2->SM
-//         8.2 TB/s at 40 % tensor-pipe activity in MODE 1, 57 % in MODE 2).
-// MODE 3: the same two CTAs as a tcgen05 CTA PAIR (cta_group::2): the leader issues ONE 256 x BN x 8 MMA for both SMs, each
-//         CTA keeps only its half of the weight tile (no multicast copy), so shared-memory operand reads per SM drop from
-//         (128 + BN) to (128 + BN/2) rows per MMA and the stage ring deepens from 4 to 6 slabs in the same 192 KB.
-template <int NB, bool TAILS, int MODE>
+// Clusters of two CTAs on neighbouring 128-row blocks walk the same weight tiles in lockstep; each loads HALF of every weight
+// slab and multicasts it into both CTAs' shared memory (halves the L2 -> SM weight stream; ncu: L2->SM 8.2 TB/s at 40 %
+// tensor-pipe activity with one CTA per row block, 57 % with the cluster).  A trailing odd row block is paired with an
+// out-of-range one (all-zero A, no stores).
+template <int NB, bool TAILS>
 __global__ void __launch_bounds__(FUSED_THREADS, 1)
 rq_coupling_final_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_constant__ CUtensorMap map_a_lo,
                          const __grid_constant__ CUtensorMap map_w_hi, const __grid_constant__ CUtensorMap map_w_lo,
@@ -88,26 +80,21 @@ rq_coupling_final_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __g
                          const __grid_constant__ CUtensorMap map_yl, const FusedParams p) {
     using Cfg = FusedCfg<NB, TAILS>;
     constexpr int MP = Cfg::MP, FPT = Cfg::FPT, HC = Cfg::HALF_COLS, BN = Cfg::BN, TILE = Cfg::TILE_COLS;
-    constexpr bool PAIR = MODE == 3;
-    constexpr int CL = MODE == 1 ? 1 : 2;
-    constexpr int NST = PAIR ? PAIR_STAGES : STAGES;                 // slabs in the shared-memory ring
-    constexpr int SB = PAIR ? PAIR_STAGE_BYTES : STAGE_BYTES;        // bytes per slab: [A hi | A lo | W hi | W lo]
-    constexpr int WLO = 2 * A_BYTES + (PAIR ? B_BYTES / 2 : B_BYTES);   // offset of the W lo part inside a slab
-    static_assert(NST * SB <= STAGES * STAGE_BYTES, "ring must fit the launch's dynamic shared memory");
+    constexpr int CL = 2;                                            // CTAs per cluster
 
     extern __shared__ uint8_t smem_raw[];
     const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
     uint8_t* smem_gen = smem_raw + (smem_base - smem_u32(smem_raw));
     const uint32_t bars = smem_base + STAGES * STAGE_BYTES;
-    const uint32_t bar_full = bars, bar_empty = bars + 8 * NST;
-    const uint32_t bar_tfull = bars + 16 * NST, bar_tempty = bars + 16 * NST + 16;
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem_gen + STAGES * STAGE_BYTES + 16 * NST + 32);   // then bias barriers at +48, +64
+    const uint32_t bar_full = bars, bar_empty = bars + 8 * STAGES;
+    const uint32_t bar_tfull = bars + 16 * STAGES, bar_tempty = bars + 16 * STAGES + 16;
+    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem_gen + STAGES * STAGE_BYTES + 16 * STAGES + 32);   // then bias barriers at +48, +64
     float* s_lad = reinterpret_cast<float*>(smem_gen + STAGES * STAGE_BYTES + 256);       // [EWG-1][128] partial log|det|
     // the packed bias of the current / next column tile, staged by the producer with a bulk copy so the epilogue reads it
     // with ~30-cycle shared loads (ncu, r1: bias + x + column-index loads at the top of every tile, L2 latency each, were
     // 40 % of the epilogue warps' samples)
     float* s_bias = reinterpret_cast<float*>(smem_gen + STAGES * STAGE_BYTES + 256 + 512 * EWG);   // [2][BN_MAX]
-    const uint32_t bar_bfull = bars + 16 * NST + 48, bar_bempty = bars + 16 * NST + 64;
+    const uint32_t bar_bfull = bars + 16 * STAGES + 48, bar_bempty = bars + 16 * STAGES + 64;
     // transformed outputs of YG consecutive column tiles, [2 buffers][128 rows][YROW] fp32, sent out by one TMA store per
     // group: a row-per-thread st.global of 5 floats per tile touched 32 sectors per instruction with 4 useful bytes each
     constexpr int YG = Cfg::YG, YROW = Cfg::YROW;
@@ -122,19 +109,18 @@ rq_coupling_final_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __g
 
     if (tid_x == 0) {
         for (int b = 0; b < 2; ++b) { mbar_init(bar_bfull + 8 * b, 1); mbar_init(bar_bempty + 8 * b, 4 * EWG); }
-        // MODE 2: both CTAs' MMA threads release a slot (the peer multicasts into it); MODE 3: the leader's commit reaches
-        // both CTAs' barriers, and the leader's accumulator barrier collects the epilogue warps of BOTH CTAs
-        for (int s = 0; s < NST; ++s) { mbar_init(bar_full + 8 * s, 1); mbar_init(bar_empty + 8 * s, MODE == 2 ? 2 : 1); }
-        for (int a = 0; a < 2; ++a) { mbar_init(bar_tfull + 8 * a, 1); mbar_init(bar_tempty + 8 * a, (PAIR ? 2 : 1) * 4 * EWG); }
+        // both CTAs' MMA threads release a slot (the peer multicasts into it)
+        for (int s = 0; s < STAGES; ++s) { mbar_init(bar_full + 8 * s, 1); mbar_init(bar_empty + 8 * s, CL); }
+        for (int a = 0; a < 2; ++a) { mbar_init(bar_tfull + 8 * a, 1); mbar_init(bar_tempty + 8 * a, 4 * EWG); }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
         prefetch_tmap(&map_a_hi); prefetch_tmap(&map_a_lo); prefetch_tmap(&map_w_hi); prefetch_tmap(&map_w_lo);
     }
-    if (warp == 1) { if (PAIR) tmem_alloc_pair(smem_u32(tmem_slot), 512); else tmem_alloc(smem_u32(tmem_slot), 512); }
+    if (warp == 1) tmem_alloc(smem_u32(tmem_slot), 512);
     tc_fence_before();
-    if (CL > 1) cluster_sync_all(); else __syncthreads();   // peers' barriers are initialised before anyone signals them
+    cluster_sync_all();                                      // peers' barriers are initialised before anyone signals them
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
-    const int cta_rank = CL > 1 ? (int)cluster_ctarank() : 0;
+    const int cta_rank = (int)cluster_ctarank();
     const int first_block = blockIdx.x / CL, block_step = gridDim.x / CL;    // a "block" = CL neighbouring 128-row tiles
     const int num_blocks = (p.num_m_tiles + CL - 1) / CL;
     constexpr uint16_t cl_mask = (uint16_t)((1u << CL) - 1);
@@ -144,10 +130,8 @@ rq_coupling_final_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __g
         if (warp == 0) {
             // ================================================= TMA producer (one elected thread: uniform datapath, tc_common.cuh)
             if (elect_one()) {
-                // bytes counted on the slab's barrier: MODE 1/2 everything landing in THIS CTA's slab; MODE 3 both CTAs' loads
-                // (A of both + both halves of W) on the leader's barrier
-                constexpr uint32_t tx_bytes = PAIR ? 2u * (2u * A_BYTES + (uint32_t)BN * ROW_BYTES)
-                                                   : 2u * A_BYTES + 2u * (uint32_t)BN * ROW_BYTES;
+                // bytes counted on the slab's barrier: everything landing in THIS CTA's slab
+                constexpr uint32_t tx_bytes = 2u * A_BYTES + 2u * (uint32_t)BN * ROW_BYTES;
                 constexpr int WROWS = BN / CL;                                             // weight rows this CTA fetches
                 int stage = 0; uint32_t phase = 0;
                 int bslot = 0; uint32_t bphase = 0;
@@ -165,94 +149,67 @@ rq_coupling_final_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __g
                         for (int ks = 0; ks < num_k; ++ks) {
                             mbar_wait(bar_empty + 8 * stage, phase ^ 1);      // every CTA of the cluster has released the slot
                             const uint32_t full = bar_full + 8 * stage;
-                            const uint32_t sa = smem_base + stage * SB;
-                            if (PAIR) {
-                                const uint32_t lead = mapa_rank(full, 0);
-                                if (cta_rank == 0) mbar_expect_tx(full, tx_bytes);
-                                tma_load_2d_pair(sa, &map_a_hi, lead, ks * BK, m * BM);
-                                tma_load_2d_pair(sa + A_BYTES, &map_a_lo, lead, ks * BK, m * BM);
-                                tma_load_2d_pair(sa + 2 * A_BYTES, &map_w_hi, lead, ks * BK, n * TILE + cta_rank * WROWS);
-                                tma_load_2d_pair(sa + WLO, &map_w_lo, lead, ks * BK, n * TILE + cta_rank * WROWS);
-                                if (++stage == NST) { stage = 0; phase ^= 1; }
-                                continue;
-                            }
+                            const uint32_t sa = smem_base + stage * STAGE_BYTES;   // [A hi | A lo | W hi | W lo]
                             mbar_expect_tx(full, tx_bytes);
                             tma_load_2d(sa, &map_a_hi, full, ks * BK, m * BM);
                             tma_load_2d(sa + A_BYTES, &map_a_lo, full, ks * BK, m * BM);
-                            if (CL == 1) {
-                                tma_load_2d(sa + 2 * A_BYTES, &map_w_hi, full, ks * BK, n * TILE);
-                                tma_load_2d(sa + 2 * A_BYTES + B_BYTES, &map_w_lo, full, ks * BK, n * TILE);
-                            } else {
-                                const uint32_t off = (uint32_t)cta_rank * WROWS * ROW_BYTES;
-                                tma_load_2d_multicast(sa + 2 * A_BYTES + off, &map_w_hi, full, ks * BK, n * TILE + cta_rank * WROWS, cl_mask);
-                                tma_load_2d_multicast(sa + 2 * A_BYTES + B_BYTES + off, &map_w_lo, full, ks * BK,
-                                                      n * TILE + cta_rank * WROWS, cl_mask);
-                            }
-                            if (++stage == NST) { stage = 0; phase ^= 1; }
+                            const uint32_t off = (uint32_t)cta_rank * WROWS * ROW_BYTES;
+                            tma_load_2d_multicast(sa + 2 * A_BYTES + off, &map_w_hi, full, ks * BK, n * TILE + cta_rank * WROWS, cl_mask);
+                            tma_load_2d_multicast(sa + 2 * A_BYTES + B_BYTES + off, &map_w_lo, full, ks * BK,
+                                                  n * TILE + cta_rank * WROWS, cl_mask);
+                            if (++stage == STAGES) { stage = 0; phase ^= 1; }
                         }
                     }
                 }
             }
-        } else if (warp == 1 && (!PAIR || cta_rank == 0)) {
-            // ================================================= MMA issuer: one partial sum per DRAIN_SLABS_FUSED slabs.  The whole warp
-            // runs the loop (stage indices / descriptors stay uniform); only lane 0 issues tcgen05.mma / tcgen05.commit.
+        } else if (warp == 1) {
+            // ================================================= MMA issuer: one partial sum per DRAIN_SLABS_FUSED slabs
             if (elect_one()) {                       // one elected thread runs the role (uniform datapath, tc_common.cuh: elect_one)
-                const bool leader = true;
-                const uint32_t idesc = make_idesc(BN, PAIR ? 2 * BM : BM);
+                const uint32_t idesc = make_idesc(BN);
                 int stage = 0; uint32_t phase = 0;
                 int acc = 0; uint32_t acc_phase = 0;
-                auto mma = [&](uint32_t d, uint64_t a, uint64_t b, uint32_t accumulate) {
-                    if (!leader) return;
-                    if (PAIR) umma_f16_pair(d, a, b, idesc, accumulate); else umma_f16(d, a, b, idesc, accumulate);
-                };
                 for (int mb = first_block; mb < num_blocks; mb += block_step) {
                     for (int n = 0; n < p.num_n_tiles; ++n) {
                         for (int g = 0; g < num_groups; ++g) {
                             // one partial sum = DRAIN_SLABS_FUSED resident K-slabs; every small cross term (lo*hi, hi*lo) is
                             // issued before the first main product, so only the main MMAs round at full magnitude
                             const int slabs = min(DRAIN_SLABS_FUSED, num_k - g * DRAIN_SLABS_FUSED);
-                            if (PAIR) mbar_wait_cluster(bar_tempty + 8 * acc, acc_phase ^ 1);
-                            else mbar_wait(bar_tempty + 8 * acc, acc_phase ^ 1);
+                            mbar_wait(bar_tempty + 8 * acc, acc_phase ^ 1);
                             const uint32_t d_tmem = tmem_base + acc * BN_MAX;
                             for (int j0 = 0; j0 < slabs; j0 += 2) {           // pairs of resident slabs: cross terms of both, then mains
                                 const int pair = min(2, slabs - j0);
                                 int st = stage; uint32_t ph = phase;
                                 for (int j = 0; j < pair; ++j) {
                                     mbar_wait(bar_full + 8 * st, ph);
-                                    if (++st == NST) { st = 0; ph ^= 1; }
+                                    if (++st == STAGES) { st = 0; ph ^= 1; }
                                 }
                                 tc_fence_after();
                                 st = stage;
                                 for (int j = 0; j < pair; ++j) {
-                                    const uint32_t sa = smem_base + st * SB;
+                                    const uint32_t sa = smem_base + st * STAGE_BYTES;
                                     const uint64_t a_hi = make_smem_desc(sa), a_lo = make_smem_desc(sa + A_BYTES);
-                                    const uint64_t w_hi = make_smem_desc(sa + 2 * A_BYTES), w_lo = make_smem_desc(sa + WLO);
+                                    const uint64_t w_hi = make_smem_desc(sa + 2 * A_BYTES), w_lo = make_smem_desc(sa + 2 * A_BYTES + B_BYTES);
 #pragma unroll
                                     for (int kk = 0; kk < BK / 16; ++kk) {
                                         const uint64_t adv = (uint64_t)(kk * 2);
-                                        mma(d_tmem, a_lo + adv, w_hi + adv, (j0 | j | kk) != 0);
-                                        mma(d_tmem, a_hi + adv, w_lo + adv, 1);
+                                        umma_f16(d_tmem, a_lo + adv, w_hi + adv, idesc, (j0 | j | kk) != 0);
+                                        umma_f16(d_tmem, a_hi + adv, w_lo + adv, idesc, 1);
                                     }
-                                    if (++st == NST) st = 0;
+                                    if (++st == STAGES) st = 0;
                                 }
                                 for (int j = 0; j < pair; ++j) {
-                                    const uint32_t sa = smem_base + stage * SB;
+                                    const uint32_t sa = smem_base + stage * STAGE_BYTES;
                                     const uint64_t a_hi = make_smem_desc(sa), w_hi = make_smem_desc(sa + 2 * A_BYTES);
 #pragma unroll
                                     for (int kk = 0; kk < BK / 16; ++kk) {
                                         const uint64_t adv = (uint64_t)(kk * 2);
-                                        mma(d_tmem, a_hi + adv, w_hi + adv, 1);
+                                        umma_f16(d_tmem, a_hi + adv, w_hi + adv, idesc, 1);
                                     }
-                                    if (!leader) {}
-                                    else if (MODE == 1) umma_commit(bar_empty + 8 * stage);
-                                    else if (MODE == 2) umma_commit_multicast(bar_empty + 8 * stage, cl_mask);   // releases the slot in every CTA
-                                    else umma_commit_pair(bar_empty + 8 * stage, cl_mask);
-                                    if (++stage == NST) { stage = 0; phase ^= 1; }
+                                    umma_commit_multicast(bar_empty + 8 * stage, cl_mask);   // releases the slot in every CTA
+                                    if (++stage == STAGES) { stage = 0; phase ^= 1; }
                                 }
                             }
-                            if (!leader) {}
-                            else if (PAIR) umma_commit_pair(bar_tfull + 8 * acc, cl_mask);   // both CTAs' halves of the sum are complete
-                            else umma_commit(bar_tfull + 8 * acc);
+                            umma_commit(bar_tfull + 8 * acc);
                             if (++acc == 2) { acc = 0; acc_phase ^= 1; }
                         }
                     }
@@ -319,10 +276,7 @@ rq_coupling_final_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __g
                     }
                     tc_fence_before();
                     __syncwarp();
-                    if (lane == 0) {
-                        if (PAIR) mbar_arrive_cluster(mapa_rank(bar_tempty + 8 * acc, 0));   // the leader's MMA thread reuses the accumulator
-                        else mbar_arrive(bar_tempty + 8 * acc);
-                    }
+                    if (lane == 0) mbar_arrive(bar_tempty + 8 * acc);
                     if (++acc == 2) { acc = 0; acc_phase ^= 1; }
                 }
                 if (n + 1 < p.num_n_tiles) load_x(n + 1, xin_next, col_next);
@@ -440,27 +394,15 @@ rq_coupling_final_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __g
     }
 
     tc_fence_before();
-    if (CL > 1) cluster_sync_all(); else __syncthreads();   // no CTA exits while a peer may still signal its barriers
-    if (warp == 1) { if (PAIR) tmem_dealloc_pair(tmem_base, 512); else tmem_dealloc(tmem_base, 512); }
+    cluster_sync_all();                                      // no CTA exits while a peer may still signal its barriers
+    if (warp == 1) tmem_dealloc(tmem_base, 512);
 }
 
-// NFK_CLUSTER = 1: single CTAs, 3: CTA pairs (cta_group::2), anything else / unset: multicast clusters.  Measured (ms per
-// step in this kernel, cfg 3): mode 2 263, mode 3 288 -- with the GPU at its power cap (sw_power_cap, ~1.78 GHz) the pair's
-// lock-step accumulator hand-off costs more than the halved shared-memory operand traffic returns.
-static int cluster_mode() {
-    static int mode = 0;
-    if (!mode) {
-        const char* e = getenv("NFK_CLUSTER");
-        mode = (e && e[0] == '1') ? 1 : (e && e[0] == '3') ? 3 : 2;
-    }
-    return mode;
-}
-
-template <int NB, bool TAILS, int MODE>
-static int launch_fused_cl(const CUtensorMap& ma_hi, const CUtensorMap& ma_lo, const __half* w_hi, const __half* w_lo, int64_t ldw,
-                           FusedParams& p, cudaStream_t st, __half* pair_hi, __half* pair_lo, int64_t pair_lds) {
+template <int NB, bool TAILS>
+static int launch_fused(const CUtensorMap& ma_hi, const CUtensorMap& ma_lo, const __half* w_hi, const __half* w_lo, int64_t ldw,
+                        FusedParams& p, cudaStream_t st, __half* pair_hi, __half* pair_lo, int64_t pair_lds) {
     using Cfg = FusedCfg<NB, TAILS>;
-    constexpr int CL = MODE == 1 ? 1 : 2;
+    constexpr int CL = 2;
     const int packed_rows = p.d_t * Cfg::MP;
     CUtensorMap mw_hi, mw_lo;
     int rc;
@@ -483,7 +425,7 @@ static int launch_fused_cl(const CUtensorMap& ma_hi, const CUtensorMap& ma_lo, c
     static DeviceOnce attr_once;
     int attr_dev = 0;
     if (attr_once.pending(&attr_dev)) {
-        cudaError_t e = cudaFuncSetAttribute(rq_coupling_final_kernel<NB, TAILS, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+        cudaError_t e = cudaFuncSetAttribute(rq_coupling_final_kernel<NB, TAILS>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
         if (e != cudaSuccess) return fail(NFK_E_CUDA, "cudaFuncSetAttribute(smem=%d): %s", smem, cudaGetErrorString(e));
         attr_once.mark(attr_dev);
     }
@@ -499,19 +441,9 @@ static int launch_fused_cl(const CUtensorMap& ma_hi, const CUtensorMap& ma_lo, c
     attr[0].val.clusterDim.x = CL; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    cudaError_t e = cudaLaunchKernelEx(&cfg, rq_coupling_final_kernel<NB, TAILS, MODE>, ma_hi, ma_lo, mw_hi, mw_lo, my, myh, myl, p);
+    cudaError_t e = cudaLaunchKernelEx(&cfg, rq_coupling_final_kernel<NB, TAILS>, ma_hi, ma_lo, mw_hi, mw_lo, my, myh, myl, p);
     if (e != cudaSuccess) return fail(NFK_E_CUDA, "cudaLaunchKernelEx(rq_coupling_final_kernel, cluster %d): %s", CL, cudaGetErrorString(e));
     return check_launch("rq_coupling_final_kernel");
-}
-
-template <int NB, bool TAILS>
-static int launch_fused(const CUtensorMap& ma_hi, const CUtensorMap& ma_lo, const __half* w_hi, const __half* w_lo, int64_t ldw,
-                        FusedParams& p, cudaStream_t st, __half* pair_hi, __half* pair_lo, int64_t pair_lds) {
-    switch (cluster_mode()) {
-        case 1: return launch_fused_cl<NB, TAILS, 1>(ma_hi, ma_lo, w_hi, w_lo, ldw, p, st, pair_hi, pair_lo, pair_lds);
-        case 2: return launch_fused_cl<NB, TAILS, 2>(ma_hi, ma_lo, w_hi, w_lo, ldw, p, st, pair_hi, pair_lo, pair_lds);
-        default: return launch_fused_cl<NB, TAILS, 3>(ma_hi, ma_lo, w_hi, w_lo, ldw, p, st, pair_hi, pair_lo, pair_lds);
-    }
 }
 
 }  // namespace tc

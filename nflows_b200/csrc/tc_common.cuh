@@ -21,9 +21,6 @@ constexpr int HALF = BN_MAX / 2;     // columns per epilogue warp
 constexpr int A_BYTES = BM * BK * 2;             // 8 KB
 constexpr int B_BYTES = BN_MAX * BK * 2;         // 16 KB
 constexpr int STAGE_BYTES = 2 * A_BYTES + 2 * B_BYTES;   // 48 KB
-// CTA-pair kernels hold half of every B tile per CTA: 32 KB stages, six of them in the same 192 KB
-constexpr int PAIR_STAGE_BYTES = 2 * A_BYTES + B_BYTES;
-constexpr int PAIR_STAGES = 6;
 constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + 1024 /*alignment slack*/ + 256 /*barriers*/;
 
 // ---------------------------------------------------------------- PTX wrappers
@@ -86,9 +83,6 @@ __device__ __forceinline__ void tma_load_2d_multicast(uint32_t dst, const CUtens
 // which ptxas cannot fold away: the arrive cannot issue before the loaded registers exist, i.e. before shared memory was read.
 // (A generic->async proxy fence in front of it as well costs ~1 000 cycles per use: two per column tile and warp.)
 __device__ __forceinline__ void mbar_arrive_after_loads(uint32_t bar, uint32_t loaded_bits, uint32_t zero) {
-#ifdef NFK_RELEASE_WITH_PROXY_FENCE
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");      // r2 first fix: dependency AND fence (~1 000 cycles per fence)
-#endif
     mbar_arrive(bar + (loaded_bits & zero));
 }
 
@@ -110,60 +104,6 @@ __device__ __forceinline__ uint32_t cluster_ctarank() {
 }
 __device__ __forceinline__ void cluster_sync_all() {
     asm volatile("barrier.cluster.arrive.release.aligned;\nbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// ---- CTA-pair (cta_group::2) variants.  The two CTAs of a cluster sit on the two SMs of one TPC; ONE tcgen05.mma issued by
-// the leader (cluster rank 0) drives both tensor cores on a 256-row tile: each CTA supplies its own 128 A rows and HALF of
-// the B tile from its own shared memory, which halves the shared-memory operand traffic per SM -- the limiter of the
-// single-CTA form (A + full B read from smem for every MMA: ~97 B/clk of the SM's 128 B/clk while the pipe is busy).
-__device__ __forceinline__ uint32_t mapa_rank(uint32_t addr, uint32_t rank) {          // same smem offset in CTA `rank`
-    uint32_t r;
-    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank));
-    return r;
-}
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
-    asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
-__device__ __forceinline__ void mbar_wait_cluster(uint32_t bar, uint32_t parity) {      // acquires remote (peer CTA) arrivals
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "WAIT_%=:\n"
-        "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%0], %1;\n"
-        "@p bra DONE_%=;\n"
-        "bra WAIT_%=;\n"
-        "DONE_%=:\n"
-        "}\n" ::"r"(bar),
-        "r"(parity)
-        : "memory");
-}
-// TMA load into THIS CTA's smem whose bytes are counted on the LEADER CTA's mbarrier (`leader_bar` = mapa_rank(bar, 0))
-__device__ __forceinline__ void tma_load_2d_pair(uint32_t dst, const CUtensorMap* map, uint32_t leader_bar, int c0, int c1) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];" ::"r"(dst),
-        "l"(reinterpret_cast<uint64_t>(map)), "r"(leader_bar), "r"(c0), "r"(c1)
-        : "memory");
-}
-__device__ __forceinline__ void tmem_alloc_pair(uint32_t dst_smem, uint32_t cols) {     // one warp of EACH CTA of the pair
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(dst_smem), "r"(cols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc_pair(uint32_t taddr, uint32_t cols) {
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols) : "memory");
-}
-__device__ __forceinline__ void umma_f16_pair(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "setp.ne.b32 p, %4, 0;\n"
-        "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n"
-        "}\n" ::"r"(d_tmem),
-        "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-__device__ __forceinline__ void umma_commit_pair(uint32_t bar, uint16_t mask) {         // arrives at `bar`'s offset in every CTA of mask
-    asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
-                 "h"(mask)
-                 : "memory");
 }
 __device__ __forceinline__ void prefetch_tmap(const CUtensorMap* map) {
     asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(map)) : "memory");
@@ -195,14 +135,6 @@ __device__ __forceinline__ void umma_commit_multicast(uint32_t bar, uint16_t mas
                  "h"(mask)
                  : "memory");
 }
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&v)[16]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-        : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]),
-          "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-        : "r"(taddr)
-        : "memory");
-}
 __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
     asm volatile(
         "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
@@ -225,14 +157,10 @@ __device__ __forceinline__ uint64_t make_smem_desc(uint32_t saddr) {
     return (uint64_t)((saddr & 0x3FFFFu) >> 4) | (1ull << 16) | ((uint64_t)((8 * ROW_BYTES) >> 4) << 32) | (1ull << 46) |
            ((uint64_t)(ROW_BYTES == 128 ? 2 : 4) << 61);
 }
-// K-major operand with 32-byte rows (one K = 16 step of fp16), SWIZZLE_32B (layout type 6): 8-row groups are 256 bytes apart
-__device__ __forceinline__ uint64_t make_smem_desc_k16(uint32_t saddr) {
-    return (uint64_t)((saddr & 0x3FFFFu) >> 4) | (1ull << 16) | ((uint64_t)((8 * 32) >> 4) << 32) | (1ull << 46) | (6ull << 61);
-}
 // cute::UMMA::InstrDescriptor: c=F32 (1<<4), a=b=F16 (format 0 at [7,10) and [10,13)), K-major both, N>>3 at [17,23),
-// M>>4 at [24,29)
-__device__ __forceinline__ uint32_t make_idesc(int bn, int m = BM) {
-    return (1u << 4) | ((uint32_t)(bn >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
+// M>>4 at [24,29) (M = BM)
+__device__ __forceinline__ uint32_t make_idesc(int bn) {
+    return (1u << 4) | ((uint32_t)(bn >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);
 }
 
 
@@ -247,7 +175,6 @@ __device__ __forceinline__ void split_f16(float v, float scale, __half& hi, __ha
 
 // host helpers (nfk_linear_tc.cu)
 int make_map(CUtensorMap* map, const __half* base, int64_t rows, int K, int64_t ld, int box_rows);
-int make_map_k16(CUtensorMap* map, const __half* base, int64_t rows, int K, int64_t ld, int box_rows);
 int make_out_map(CUtensorMap* map, float* base, int64_t rows, int64_t cols, int64_t ld, int box_cols, int box_rows);
 int make_out_map16(CUtensorMap* map, __half* base, int64_t rows, int64_t cols, int64_t ld, int box_cols, int box_rows);
 int sm_count();

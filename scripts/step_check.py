@@ -94,7 +94,7 @@ def coupling(features, hidden, blocks, rows, bins=8, tails="linear", inverse=Fal
 
 
 STAGES = {
-    "t0": lambda: trunk(64, 0, 128, 40),          # initial layer only, one tile (cluster of 1 when NFK_CLUSTER=1)
+    "t0": lambda: trunk(64, 0, 128, 40),          # initial layer only, one tile
     "t1": lambda: trunk(64, 1, 130, 40),          # one residual block, two tiles
     "t2": lambda: trunk(256, 2, 1000, 40),        # cfg-3 widths
     "t3": lambda: trunk(128, 3, 4096, 392),       # long initial layer (13 K-slabs: wraps the 4-stage ring), 6 square layers

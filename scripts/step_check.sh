@@ -4,24 +4,9 @@ mkdir -p gpurun_out
 LOG=gpurun_out/step_check.log
 : > $LOG
 run() { echo "--- $*" >> $LOG; timeout 120 "$@" >> $LOG 2>&1; echo "rc=$?" >> $LOG; }
-NFK_CLUSTER=1 run python scripts/step_check.py t1
-for s in t2 t3 t4 c0 c1 c2 c3 c4 c5 c6 c7 c8; do run python scripts/step_check.py $s; done
-NFK_STEP_EWG=2 run python scripts/step_check.py c1
-NFK_STEP_EWG=2 run python scripts/step_check.py c3
+for s in t0 t1 t2 t3 t4 c0 c1 c2 c3 c4 c5 c6 c7 c8; do run python scripts/step_check.py $s; done
 echo "=== pytest gpu" >> $LOG
 timeout 900 python -m pytest tests -m gpu -q -x 2>&1 | tail -15 >> $LOG
-for v in 4 2; do
-  NFK_STEP_EWG=$v timeout 400 python bench.py --steps 5 --warmup 3 --no-cpu-baseline --no-spline-roofline --no-extras 2>gpurun_out/bench_ewg$v.err | tail -1 > gpurun_out/bench_ewg$v.json
-  python - "$v" >> $LOG <<'PY'
-import json, sys
-try:
-    d = json.load(open("gpurun_out/bench_ewg%s.json" % sys.argv[1]))
-    print("EWG", sys.argv[1], "samples/s %.0f" % d["value"], "ms/step %.1f" % d["ms_per_step"], "clk", d["clocks"]["sm_mhz"], d["timeline_ms_per_step"], "launches", d["gpu_launches"], "parity", d.get("parity_check"), "e2e", d["e2e"]["value"])
-except Exception as e:
-    print("bench failed", sys.argv[1], e)
-PY
-  tail -3 gpurun_out/bench_ewg$v.err >> $LOG
-done
 echo "=== ncu step kernel" >> $LOG
 timeout 600 ncu --set full --clock-control none --import-source on -k regex:rq_coupling_step -s 4 -c 1 -o gpurun_out/ncu_step_r2b -f python bench.py --steps 1 --warmup 1 --rows 262144 --no-cpu-baseline --no-spline-roofline --no-extras --no-parity-check 2>&1 | tail -2 >> $LOG
 cat $LOG

@@ -398,7 +398,8 @@ def test_domain_check_can_be_disabled(cuda_device):
 
 
 @torch.no_grad()
-@pytest.mark.parametrize("bins,tails", [(8, "linear"), (10, "linear"), (4, "linear"), (16, "linear"), (8, None), (10, None)])
+@pytest.mark.parametrize("bins,tails", [(8, "linear"), (10, "linear"), (4, "linear"), (16, "linear"), (8, None), (10, None),
+                                       (16, None)])
 def test_fused_coupling_kernel_matches_unfused_and_oracle(cuda_device, bins, tails, monkeypatch):
     """The one-kernel final-layer+spline path against (a) the GEMM -> HBM params -> spline-kernel path with the FFMA GEMM
     and (b) the CPU oracle, forward and inverse, ragged row count, odd feature count."""
